@@ -1,10 +1,11 @@
 #!/usr/bin/env python3
 """bench.py -- MFCC frames/s (48 kHz, n_fft=2048, hop=512, 128 mel, 40 coefficients) on N B200s.
 
-Contract (see the task statement / DESIGN.md section 6):
+Usage (DESIGN.md section 6):
   python bench.py --gpus N --steps K --warmup W            (N>1: launched under torchrun, one rank per GPU)
   python bench.py --impl reference ...                     (the reference's own CPU path, oracle/_ref)
-One JSON line on stdout from rank 0.
+  python bench.py ... --dump-outputs DIR                   (also write the MFCCs of the last timed step to DIR/mfcc.npy)
+One JSON line on stdout from rank 0.  K is the number of timed steps of every timed loop.
 
 A "step" is one pass of the fused STFT->mel->log->DCT path over one synthetic batch:
   N=1 : BASELINE config 2 = 1024 clips x 5 s (983 MB of samples, larger than the 126 MB L2).
@@ -185,6 +186,24 @@ class ClockSampler:
                 "source": "nvml" if self.nvml is not None else "nvidia-smi", "reasons": reasons}
 
 
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, arrays):
+    """Write each (clips, ...) result as out_dir/<name>.npy in float32.  A result larger than its share of DUMP_BYTES is
+    cut to a fixed sample of clips (numpy seed 0, ascending clip order), the same for every run with the same --batch /
+    --gpus, so that two builds can be compared output for output."""
+    os.makedirs(out_dir, exist_ok=True)
+    budget = DUMP_BYTES // len(arrays)
+    for name, a in arrays.items():
+        n = a.shape[0]
+        per_clip = 4 * a[0].numel()
+        if n * per_clip > budget:
+            keep = np.sort(np.random.default_rng(0).choice(n, budget // per_clip, replace=False))
+            a = a[keep]
+        np.save(os.path.join(out_dir, name + ".npy"), a.float().cpu().numpy())
+
+
 # --------------------------------------------------------------------------- reference / CPU arm
 def _cpu_worker(args):
     lib_path, seed, clips, warm = args
@@ -351,7 +370,7 @@ def run_reference_arm(args):
     per = max(2, int(os.environ.get("AFB200_CPU_CLIPS_PER_WORKER", "16")))
     vals, runs = [], []
     t_all = time.perf_counter()
-    for _ in range(max(1, min(args.steps, 3))):
+    for _ in range(args.steps):
         r = cpu_reference_rate(per, cores)
         if r is None:
             emit({"impl": "reference", "unavailable": "oracle/_ref/libaudioflux_ref.so not built"})
@@ -423,7 +442,7 @@ def bench_cqt_c3(dev, peaks, args, cores):
         return {"error": f"CQT parity gate failed: rel err {errs}"}
     del re, im
     n0 = lib.afb200_kernelLaunchCount()
-    ms = _timed_ms(lambda: c.cqt_batch(x), steps=max(3, min(args.steps, 10)), warm=3)
+    ms = _timed_ms(lambda: c.cqt_batch(x), steps=args.steps, warm=3)
     launches = (lib.afb200_kernelLaunchCount() - n0) // (len(ms) + 3)
     ms_step = float(np.mean(ms))
     # end to end: the C-ABI call with page-locked HOST buffers (chunked copy-in / transform / copy-out inside)
@@ -505,8 +524,8 @@ def bench_cwt_c4(dev, peaks, args, cores):
     if not err < 1e-4:
         return {"error": f"CWT parity gate failed: rel err {err}"}
     n0 = lib.afb200_kernelLaunchCount()
-    ms = _timed_ms(step, steps=3, warm=1)
-    launches = (lib.afb200_kernelLaunchCount() - n0) // 4
+    ms = _timed_ms(step, steps=args.steps, warm=1)
+    launches = (lib.afb200_kernelLaunchCount() - n0) // (len(ms) + 1)
     ms_step = float(np.mean(ms))
     # end to end: cwtObj_cwtBatch with HOST pointers, chunk by chunk (inputs from and planes to page-locked host memory)
     xh = torch.empty((chunk, N), dtype=torch.float32).pin_memory()
@@ -660,10 +679,16 @@ def run_b200_arm(args):
     sampler.mark(True)
     ev[0].record()
     for i in range(args.steps):
-        step()
+        last = step()
         ev[i + 1].record()
     torch.cuda.synchronize()
     sampler.mark(False)
+    if args.dump_outputs and rank == 0:
+        if scatter is not None:            # (world, B, T, cc)
+            last = last.reshape(world * B, T, NCC)
+        elif overlap is not None:          # chunk k gathered as (world * B / chunks, T, cc), rank-major inside the chunk
+            last = torch.cat([o.view(world, -1, T, NCC) for o in last], dim=1).reshape(world * B, T, NCC)
+        dump_outputs(args.dump_outputs, {"mfcc": last})
     if dist:
         dist.barrier()
     launches = lib.afb200_kernelLaunchCount() - launches0
@@ -735,7 +760,7 @@ def run_b200_arm(args):
     if dist:
         dist.barrier()
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    n_e2e = max(3, min(args.steps, 10))
+    n_e2e = args.steps
     e0.record()
     for _ in range(n_e2e):
         e2e_step()
@@ -834,8 +859,15 @@ def main():
     ap.add_argument("--gather-chunks", type=int, default=4, help="N>1, --gather nccl: chunks per step for compute/all-gather overlap")
     ap.add_argument("--gather", choices=("peer", "nccl"), default="peer",
                     help="N>1: 'peer' = all-gather fused into the kernel epilogue (NVLink P2P stores); 'nccl' = overlapped NCCL all-gather")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps write the MFCCs of the last one -- the headline path; the CQT / CWT keys "
+                         "dump nothing -- to DIR/mfcc.npy (float32; a fixed sample of clips when the batch exceeds 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
+        if args.dump_outputs:
+            ap.error("--dump-outputs writes the B200 path's MFCCs; it does not apply to --impl reference")
         return run_reference_arm(args)
     return run_b200_arm(args)
 

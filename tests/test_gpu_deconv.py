@@ -10,24 +10,30 @@ pytestmark = pytest.mark.gpu
 
 
 @pytest.mark.parametrize("num,bpo,hc", [(84, 12, 20), (96, 24, 30), (36, 12, 8)])
-def test_deconv_cqhc_vs_oracle_and_reference(cuda_device, ref_lib, num, bpo, hc):
+def test_deconv_cqhc_vs_oracle_and_reference(cuda_device, reference, num, bpo, hc):
     import audioflux_b200 as af
     x = (0.1 * np.random.default_rng(1).standard_normal(24000)).astype(np.float32)
-    c, cr = af.CQT(num, 32000, bin_per_octave=bpo), af.CQT(num, 32000, bin_per_octave=bpo, _lib=ref_lib)
-    z, zr = c.cqt(x), cr.cqt(x)
-    assert rel_max(np.abs(z), np.abs(zr)) < 1e-4
-    m = np.ascontiguousarray(np.abs(zr).T.astype(np.float32))
+    c = af.CQT(num, 32000, bin_per_octave=bpo)
+    z = c.cqt(x)
+    zr_abs = reference("cqt_abs", lambda lib: np.abs(af.CQT(num, 32000, bin_per_octave=bpo, _lib=lib).cqt(x)))
+    assert rel_max(np.abs(z), zr_abs) < 1e-4
+    m = spectra(z.shape[1], num, num + hc)        # CQT-shaped magnitudes, the same input for all three wherever the test runs
+
+    def ref(lib):
+        cr = af.CQT(num, 32000, bin_per_octave=bpo, _lib=lib)
+        cr.cqt(x)                                                  # sets the object's timeLength
+        return tuple(cr.deconv_planes(m)) + (cr.cqhc_planes(m, hc),)
+    r_tone, r_pitch, r_cqhc = reference("tone,pitch,cqhc", ref)
     tone, pitch = c.deconv_planes(m)
     o_tone, o_pitch = O.cq_deconv(m, bpo)
-    r_tone, r_pitch = cr.deconv_planes(m)
     assert rel_max(tone, o_tone) < 1e-4 and rel_max(pitch, o_pitch) < 1e-4
     assert rel_max(tone, r_tone) < 1e-4 and rel_max(pitch, r_pitch) < 1e-4
     got = c.cqhc_planes(m, hc)
-    assert rel_max(got, O.cqhc(m, hc, bpo)) < 1e-4 and rel_max(got, cr.cqhc_planes(m, hc)) < 1e-4
+    assert rel_max(got, O.cqhc(m, hc, bpo)) < 1e-4 and rel_max(got, r_cqhc) < 1e-4
     # python-layout wrappers: [num, T] in, [.., T] out
-    t2, p2 = c.deconv(np.abs(zr))
+    t2, p2 = c.deconv(np.ascontiguousarray(m.T))
     assert t2.shape == (num, m.shape[0]) and np.allclose(t2.T, tone) and np.allclose(p2.T, pitch)
-    assert c.cqhc(zr, hc).shape == (hc, m.shape[0])
+    assert c.cqhc(z, hc).shape == (hc, m.shape[0])
 
 
 def test_deconv_batch_any_rows_host_and_device(cuda_device):
@@ -46,22 +52,28 @@ def test_deconv_batch_any_rows_host_and_device(cuda_device):
 
 
 @pytest.mark.parametrize("num,scale,r", [(128, "MEL", 11), (40, "BARK", 10), (257, "LINEAR", 9)])
-def test_spectrogram_deconv_vs_oracle_and_reference(cuda_device, ref_lib, num, scale, r):
+def test_spectrogram_deconv_vs_oracle_and_reference(cuda_device, reference, num, scale, r):
     """spectrogramObj_deconv / spectrogramObj_deconvBatch: same kernel as cqtObj_deconv, band count of the spectrogram"""
     import torch
     import audioflux_b200 as af
     x = (0.1 * np.random.default_rng(3).standard_normal(12000)).astype(np.float32)
     kw = dict(radix2_exp=r, samplate=16000, filter_bank_type=getattr(af.SpectralFilterBankScaleType, scale))
-    s, q = af.Spectrogram(num, **kw), af.Spectrogram(num, _lib=ref_lib, **kw)
-    spec, spec_r = s.spectrogram(x), q.spectrogram(x)
+    s = af.Spectrogram(num, **kw)
+    spec = s.spectrogram(x)
+
+    def ref(lib):
+        q = af.Spectrogram(num, _lib=lib, **kw)
+        spec_r = q.spectrogram(x)                      # also sets the object's timeLength
+        return (spec_r,) + tuple(q.deconv(np.ascontiguousarray(spectra(spec_r.shape[1], num, num + r).T)))
+    spec_r, r_tone, r_pitch = reference("spec,tone,pitch", ref)
     assert rel_max(spec, spec_r) < 1e-4
-    tone, pitch = s.deconv(spec_r)                     # same input for all three
-    r_tone, r_pitch = q.deconv(spec_r)
-    o_tone, o_pitch = O.cq_deconv(np.ascontiguousarray(spec_r.T))
-    assert tone.shape == spec_r.shape
+    spec = np.ascontiguousarray(spectra(spec.shape[1], num, num + r).T)    # [num, T], the same input for all three
+    tone, pitch = s.deconv(spec)
+    o_tone, o_pitch = O.cq_deconv(np.ascontiguousarray(spec.T))
+    assert tone.shape == spec.shape
     assert rel_max(tone.T, o_tone) < 1e-4 and rel_max(pitch.T, o_pitch) < 1e-4
     assert rel_max(tone, r_tone) < 1e-4 and rel_max(pitch, r_pitch) < 1e-4
-    m = np.ascontiguousarray(np.stack([spec_r.T, 2.0 * spec_r.T]))            # [2, T, num]
+    m = np.ascontiguousarray(np.stack([spec.T, 2.0 * spec.T]))                # [2, T, num]
     bt, bp = s.deconv_batch(m)
     assert np.array_equal(bt[0], tone.T) and rel_max(bt[1], 2.0 * tone.T) < 1e-5
     dt, dp = s.deconv_batch(torch.from_numpy(m).cuda())

@@ -7,7 +7,7 @@ import numpy as np
 import pytest
 
 import audioflux_b200 as af
-from conftest import noise, rel_max, tones
+from conftest import noise, ref_absmax, ref_pair, rel_max, tones
 from oracle import af_oracle as O
 from test_next_rows_cpu import SPEC_CASES, _phase_mask
 
@@ -172,24 +172,30 @@ def test_spectrogram_mfcc_batch_is_the_fused_kernel(torch_cuda, golden):
     assert rel_max(mel[0].cpu().numpy(), g["mel"]) < TOL
 
 
-def test_next_rows_against_reference_build(torch_cuda, ref_lib):
-    """Same calls into oracle/_ref (the unmodified reference) and into libaudioflux_b200."""
+def test_next_rows_against_reference_build(torch_cuda, reference):
+    """Same calls into oracle/_ref (the unmodified reference, or its stored results) and into libaudioflux_b200."""
     x = tones(21, 24000, 32000)
-    for kw in SPEC_CASES[:8]:
+    for i, kw in enumerate(SPEC_CASES[:8]):
         xr = tones(22, 24000, kw["samplate"])
-        a, r = af.Spectrogram(**kw), af.Spectrogram(_lib=ref_lib, **kw)
-        assert rel_max(a.spectrogram_planes(xr), r.spectrogram_planes(xr)) < TOL
-    qa, qr = af.CQT(84, 32000), af.CQT(84, 32000, _lib=ref_lib)
-    ra, ia = qa.cqt_planes(x)
-    rr, ir = qr.cqt_planes(x)
-    assert rel_max(qa.chroma_planes(ra, ia), qr.chroma_planes(rr, ir)) < 2e-4
-    pr = rr * rr + ir * ir
-    assert rel_max(qa.cqcc_planes(pr, 13), qr.cqcc_planes(pr, 13)) < TOL
+        want = reference(f"spec{i}", lambda lib: af.Spectrogram(_lib=lib, **kw).spectrogram_planes(xr))
+        assert rel_max(af.Spectrogram(**kw).spectrogram_planes(xr), want) < TOL
+    # the cqcc input: the oracle's CQT power, regenerated identically wherever the test runs
+    o_re, o_im = O.cqt(x, 84, 32000)
+    pr = np.ascontiguousarray(o_re * o_re + o_im * o_im, np.float32)
+
+    def cqt(lib):
+        q = af.CQT(84, 32000, _lib=lib)
+        rr, ir = q.cqt_planes(x)                       # also sets the object's timeLength
+        assert rr.shape == pr.shape
+        return q.chroma_planes(rr, ir), q.cqcc_planes(pr, 13)
+    (chroma_a, cqcc_a), (chroma_r, cqcc_r) = cqt(None), reference("chroma,cqcc", cqt)
+    assert rel_max(chroma_a, chroma_r) < 2e-4
+    assert rel_max(cqcc_a, cqcc_r) < TOL
     m = (np.random.default_rng(5).random((30, 40)) * 4).astype(np.float32)
     e = (np.random.default_rng(6).random(30) * 2).astype(np.float32)
     for et in (0, 1, 2):
-        for a, r in zip(af.XXCC(40).xxcc_standard_planes(m, e, 13, 9, et),
-                        af.XXCC(40, _lib=ref_lib).xxcc_standard_planes(m, e, 13, 9, et)):
+        want = reference(f"xxcc_standard{et}", lambda lib: af.XXCC(40, _lib=lib).xxcc_standard_planes(m, e, 13, 9, et))
+        for a, r in zip(af.XXCC(40).xxcc_standard_planes(m, e, 13, 9, et), want):
             assert rel_max(a, r) < TOL
 
 
@@ -216,16 +222,18 @@ def test_stft_padding_modes(torch_cuda, pos, mode, v1, v2, L, n, hop):
     assert np.abs(bim[0].cpu().numpy() - im2[:, :n // 2 + 1]).max() <= TOL * scale
 
 
-def test_stft_padding_against_reference_build(torch_cuda, ref_lib):
+def test_stft_padding_against_reference_build(torch_cuda, reference):
     x = tones(63, 5000, 16000)
     for pos in (0, 1, 2):
         for mode in (0, 1, 2):
-            a, r = af.STFT(9, af.WindowType.HAMM, 128), af.STFT(9, af.WindowType.HAMM, 128, _lib=ref_lib)
-            for s in (a, r):
+            def stft(lib):
+                s = af.STFT(9, af.WindowType.HAMM, 128, _lib=lib)
                 s.enable_padding(True)
                 s.set_padding(pos, mode, 1.25, -0.75)
-            (ar, ai), (rr, ri) = a.stft_planes(x), r.stft_planes(x)
-            scale = max(np.abs(rr).max(), np.abs(ri).max())
+                return s.stft_planes(x)
+            (ar, ai), (rr, ri) = stft(None), reference(f"stft{pos}{mode}", stft)
+            scale = max(ref_absmax(rr), ref_absmax(ri))
+            (ar, rr), (ai, ri) = ref_pair(ar, rr), ref_pair(ai, ri)
             assert np.abs(ar - rr).max() <= TOL * scale and np.abs(ai - ri).max() <= TOL * scale
 
 
@@ -311,14 +319,21 @@ def test_istft(torch_cuda, r, hop, wt, method):
     assert np.abs(buf - want2)[ok].max() <= TOL * np.abs(want2).max()
 
 
-def test_istft_against_reference_build(torch_cuda, ref_lib):
+def test_istft_against_reference_build(torch_cuda, reference):
     x = tones(84, 6000, 16000)
     for wt, method in ((1, 0), (2, 1), (0, 0)):
-        a, r = af.STFT(9, wt, 128), af.STFT(9, wt, 128, _lib=ref_lib)
-        re, im = r.stft_planes(x)
-        ya, yr = a.istft_planes(re, im, method), r.istft_planes(re, im, method)
-        ok = istft_conditioned(512, 128, re.shape[0], O.fft_window(wt, 512), method)
-        assert np.abs(ya - yr)[ok].max() <= TOL * np.abs(yr).max()
+        # the same STFT planes (the oracle's, regenerated wherever the test runs) go into both inverses
+        re, im = (np.ascontiguousarray(p, np.float32) for p in O.stft(x, 512, 128, O.fft_window(wt, 512)))
+
+        def istft(lib):
+            s = af.STFT(9, wt, 128, _lib=lib)
+            assert s.stft_planes(x)[0].shape == re.shape
+            return s.istft_planes(re, im, method)
+        ya, yr = istft(None), reference(f"istft{wt}{method}", istft)
+        ok = ref_pair(istft_conditioned(512, 128, re.shape[0], O.fft_window(wt, 512), method), yr)[0]
+        scale = ref_absmax(yr)
+        ya, yr = ref_pair(ya, yr)
+        assert np.abs(ya - yr)[ok].max() <= TOL * scale
 
 
 # ------------------------------------------------------------------ PWT
@@ -349,11 +364,12 @@ def test_pwt_vs_oracle(torch_cuda, kw):
     assert np.abs(dr - d2).max() <= TOL * sd and np.abs(di - e2).max() <= TOL * sd
 
 
-def test_pwt_long_clip_and_reference_build(torch_cuda, ref_lib):
+def test_pwt_long_clip_and_reference_build(torch_cuda, reference):
     x = tones(93, 1 << 14, 32000)
-    a, r = af.PWT(84, 14, 32000, is_padding=False), af.PWT(84, 14, 32000, is_padding=False, _lib=ref_lib)
-    (ar, ai), (rr, ri) = a.pwt_planes(x), r.pwt_planes(x)
-    scale = max(np.abs(rr).max(), np.abs(ri).max())
+    ar, ai = af.PWT(84, 14, 32000, is_padding=False).pwt_planes(x)
+    rr, ri = reference("pwt", lambda lib: af.PWT(84, 14, 32000, is_padding=False, _lib=lib).pwt_planes(x))
+    scale = max(ref_absmax(rr), ref_absmax(ri))
+    (ar, rr), (ai, ri) = ref_pair(ar, rr), ref_pair(ai, ri)
     assert np.abs(ar - rr).max() <= TOL * scale and np.abs(ai - ri).max() <= TOL * scale
 
 
@@ -420,16 +436,19 @@ def test_cqt_streaming_matches_oracle_and_reference(cuda_device, ref_lib, chunks
 
 @pytest.mark.parametrize("num,sr,beta,norm,bpo", [(84, 32000, 5.0, 0, 12), (48, 44100, 2.0, 1, 12), (72, 22050, 10.0, 2, 12),
                                                    (48, 16000, 3.0, 0, 24)])
-def test_vqt_vs_oracle_and_reference(cuda_device, ref_lib, num, sr, beta, norm, bpo):
+def test_vqt_vs_oracle_and_reference(cuda_device, reference, num, sr, beta, norm, bpo):
     """VQT (beta != 0, VERDICT r1 missing #5): per-octave kernel sets through the tcgen05 / mma / FP32 octave kernels"""
     import audioflux_b200 as af
     x = (0.1 * np.random.default_rng(3).standard_normal(30000)).astype(np.float32)
     kw = dict(bin_per_octave=bpo, beta=beta, normal_type=af.SpectralFilterBankNormalType(norm))
     z = af.CQT(num, sr, **kw).cqt(x)
-    zr = af.CQT(num, sr, _lib=ref_lib, **kw).cqt(x)
+    def vqt(lib):
+        zr = af.CQT(num, sr, _lib=lib, **kw).cqt(x)
+        return np.ascontiguousarray(zr.real), np.ascontiguousarray(zr.imag)
+    zr_re, zr_im = reference("vqt", vqt)
     re, im = O.cqt(x, num, sr, bpo=bpo, beta=beta, norm=norm)
     assert rel_max(z.real, re.T) < 1e-4 and rel_max(z.imag, im.T) < 1e-4
-    assert rel_max(z.real, zr.real) < 1e-4 and rel_max(z.imag, zr.imag) < 1e-4
+    assert rel_max(z.real, zr_re) < 1e-4 and rel_max(z.imag, zr_im) < 1e-4
 
 
 def test_istft_16384_round_trip(torch_cuda):

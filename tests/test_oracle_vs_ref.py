@@ -1,12 +1,12 @@
-"""Pins the numpy restatement (oracle/af_oracle.py) to the reference compiled in oracle/_ref.
-Skipped where that library is absent."""
+"""Pins the numpy restatement (oracle/af_oracle.py) to the reference compiled in oracle/_ref.  The tests that take the
+`reference` fixture read the reference's stored results (tests/golden/ref) where that library is absent; the others skip."""
 import ctypes as C
 
 import numpy as np
 import pytest
 
 import audioflux_b200 as af
-from conftest import noise, rel_max
+from conftest import noise, ref_pair, ref_window, rel_max
 from oracle import af_oracle as O
 
 S, ST, N, D, W = (af.SpectralFilterBankScaleType, af.SpectralFilterBankStyleType,
@@ -14,11 +14,11 @@ S, ST, N, D, W = (af.SpectralFilterBankScaleType, af.SpectralFilterBankStyleType
 
 
 @pytest.mark.parametrize("wt", range(14))
-def test_windows(ref_lib, wt):
+def test_windows(reference, wt):
     for n in (16, 512, 2048):
-        p = ref_lib.window_calFFTWindow(wt, n)
-        w = np.ctypeslib.as_array(C.cast(p, C.POINTER(C.c_float)), shape=(n,)).copy()
-        assert np.abs(w - O.fft_window(wt, n)).max() < 2e-6
+        w = reference(f"window{n}", lambda lib: ref_window(lib, wt, n))
+        o, w = ref_pair(O.fft_window(wt, n), w)
+        assert np.abs(w - o).max() < 2e-6
 
 
 def _ref_bank(ref, num, n, sr, scale, style, norm, low, high, bpo):
@@ -56,9 +56,9 @@ def test_filter_banks(ref_lib, scale, style, norm):
 
 
 @pytest.mark.parametrize("r,hop,wt", [(11, 512, 1), (9, 100, 2), (10, 1024, 0), (12, 1000, 4)])
-def test_stft(ref_lib, r, hop, wt):
+def test_stft(reference, r, hop, wt):
     x = noise(1, 20000)
-    re, im = af.STFT(r, W(wt), hop, _lib=ref_lib).stft_planes(x)
+    re, im = reference("stft", lambda lib: af.STFT(r, W(wt), hop, _lib=lib).stft_planes(x))
     re2, im2 = O.stft(x, 1 << r, hop, O.fft_window(wt, 1 << r))
     assert rel_max(re2, re) < 2e-6 and rel_max(im2, im) < 2e-6
 
@@ -66,14 +66,18 @@ def test_stft(ref_lib, r, hop, wt):
 @pytest.mark.parametrize("scale,style,norm,dt,rt,nv", [
     (2, 0, 0, 0, 1, 1.0), (2, 0, 1, 1, 1, 1.0), (3, 1, 0, 0, 1, 0.5), (4, 0, 2, 1, 1, 2.0), (2, 0, 0, 0, 0, 1.0),
     (3, 0, 1, 1, 0, 1.0), (0, 0, 0, 0, 1, 1.0), (0, 0, 0, 1, 0, 1.0), (5, 0, 0, 0, 1, 1.0), (6, 1, 1, 1, 1, 1.0)])
-def test_bft_modes(ref_lib, scale, style, norm, dt, rt, nv):
+def test_bft_modes(reference, scale, style, norm, dt, rt, nv):
     x = noise(2, 20000)
     kw = dict(low_fre=32.703196, high_fre=16000.) if scale == 6 else {}
-    b = af.BFT(64, 10, 44100, slide_length=256, scale_type=S(scale), style_type=ST(style), normal_type=N(norm),
-               data_type=D(dt), _lib=ref_lib, **kw)
-    if nv != 1.0:
-        b.set_data_norm_value(nv)
-    re, im = b.bft_planes(x, rt)
+
+    def ref(lib):
+        b = af.BFT(64, 10, 44100, slide_length=256, scale_type=S(scale), style_type=ST(style), normal_type=N(norm),
+                   data_type=D(dt), _lib=lib, **kw)
+        if nv != 1.0:
+            b.set_data_norm_value(nv)
+        re, im = b.bft_planes(x, rt)
+        return (re,) if rt == 1 else (re, im)
+    re, im = (reference("bft", ref) + (None,))[:2]
     o = O.bft(x, 64, 10, 44100, 256, 1, scale, style, norm, dt, low=32.703196 if scale in (5, 6) else None,
               high=kw.get("high_fre"), result_type=rt, norm_value=nv)
     if rt == 1:
@@ -82,38 +86,43 @@ def test_bft_modes(ref_lib, scale, style, norm, dt, rt, nv):
         assert rel_max(o[0], re) < 2e-5 and rel_max(o[1], im) < 2e-5
 
 
-def test_xxcc(ref_lib):
+def test_xxcc(reference):
     m = np.abs(noise(3, 50 * 128).reshape(50, 128)) + 1e-9
     m[3, :5] = 0.0
-    x = af.XXCC(128, _lib=ref_lib)
-    assert np.abs(x.xxcc_planes(m, 40) - O.xxcc(m, 40)).max() < 2e-5
-    x2 = af.XXCC(60, _lib=ref_lib)          # non power of two -> dense DCT in the reference
-    assert np.abs(x2.xxcc_planes(m[:, :60], 13) - O.xxcc(m[:, :60], 13)).max() < 2e-5
-    assert np.abs(x.xxcc_planes(m, 20, af.CepstralRectifyType.CUBIC_ROOT) - O.xxcc(m, 20, O.RECT_CUBIC)).max() < 2e-5
+
+    def ref(lib):
+        x, x2 = af.XXCC(128, _lib=lib), af.XXCC(60, _lib=lib)    # 60: not a power of two -> dense DCT in the reference
+        return x.xxcc_planes(m, 40), x2.xxcc_planes(m[:, :60], 13), x.xxcc_planes(m, 20, af.CepstralRectifyType.CUBIC_ROOT)
+    for want, got in zip(reference("xxcc", ref), (O.xxcc(m, 40), O.xxcc(m[:, :60], 13), O.xxcc(m, 20, O.RECT_CUBIC))):
+        g, w = ref_pair(got, want)
+        assert np.abs(g - w).max() < 2e-5
 
 
-def test_decimator(ref_lib):
+def test_decimator(reference):
     x = noise(4, 20001)
-    ro = C.c_void_p()
-    ref_lib.resampleObj_new.argtypes = [C.POINTER(C.c_void_p), C.POINTER(C.c_int), C.POINTER(C.c_int), C.POINTER(C.c_int)]
-    ref_lib.resampleObj_new(C.byref(ro), C.byref(C.c_int(2)), C.byref(C.c_int(1)), None)
-    ref_lib.resampleObj_setSamplate.argtypes = [C.c_void_p, C.c_int, C.c_int]
-    ref_lib.resampleObj_setSamplate(ro, 2, 1)
-    ref_lib.resampleObj_resample.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p]
-    ref_lib.resampleObj_resample.restype = C.c_int
-    out = np.zeros(len(x), np.float32)
-    n = ref_lib.resampleObj_resample(ro, x.ctypes.data, len(x), out.ctypes.data)
+
+    def ref(lib):
+        ro = C.c_void_p()
+        lib.resampleObj_new.argtypes = [C.POINTER(C.c_void_p), C.POINTER(C.c_int), C.POINTER(C.c_int), C.POINTER(C.c_int)]
+        lib.resampleObj_new(C.byref(ro), C.byref(C.c_int(2)), C.byref(C.c_int(1)), None)
+        lib.resampleObj_setSamplate.argtypes = [C.c_void_p, C.c_int, C.c_int]
+        lib.resampleObj_setSamplate(ro, 2, 1)
+        lib.resampleObj_resample.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p]
+        lib.resampleObj_resample.restype = C.c_int
+        out = np.zeros(len(x), np.float32)
+        n = lib.resampleObj_resample(ro, x.ctypes.data, len(x), out.ctypes.data)
+        return np.array(n), out[:n]
+    n, out = reference("resample", ref)
     y = O.resample_down2(x)
     assert n == len(y) == len(x) // 2
-    assert rel_max(y, out[:n]) < 2e-6
+    assert rel_max(y, out) < 2e-6
 
 
 @pytest.mark.parametrize("L,sr,norm,hop,scale", [(48037, 48000, 1, None, True), (30000, 32000, 0, None, True),
                                                   (22050, 22050, 2, 64, False)])
-def test_cqt(ref_lib, L, sr, norm, hop, scale):
+def test_cqt(reference, L, sr, norm, hop, scale):
     x = noise(5, L)
-    c = af.CQT(84, sr, normal_type=N(norm), slide_length=hop, is_scale=scale, _lib=ref_lib)
-    re, im = c.cqt_planes(x)
+    re, im = reference("cqt", lambda lib: af.CQT(84, sr, normal_type=N(norm), slide_length=hop, is_scale=scale, _lib=lib).cqt_planes(x))
     re2, im2 = O.cqt(x, 84, sr, norm=norm, hop=hop, is_scale=scale)
     assert rel_max(re2, re) < 1e-5 and rel_max(im2, im) < 1e-5
 
@@ -121,13 +130,13 @@ def test_cqt(ref_lib, L, sr, norm, hop, scale):
 @pytest.mark.parametrize("r,wav,scale,pad", [(12, 1, 5, False), (12, 0, 5, False), (12, 2, 5, False), (11, 3, 5, False),
                                              (11, 4, 5, False), (11, 5, 5, False), (11, 6, 5, False), (11, 7, 5, False),
                                              (12, 1, 2, False), (12, 0, 3, False), (12, 1, 5, True), (10, 1, 0, False)])
-def test_cwt(ref_lib, r, wav, scale, pad):
+def test_cwt(reference, r, wav, scale, pad):
     x = noise(6, 1 << r)
     kw = dict(low_fre=1000.) if scale == 0 else {}
-    w = af.CWT(40 if scale == 0 else 84, r, 48000, wavelet_type=af.WaveletContinueType(wav), scale_type=S(scale),
-               is_padding=pad, _lib=ref_lib, **kw)
-    re, im = w.cwt_planes(x)
-    re2, im2 = O.cwt(x, w.num, r, 48000, wav, scale, low=kw.get("low_fre", 32.703196 if scale in (5, 6) else None), is_pad=pad)
+    num = 40 if scale == 0 else 84
+    re, im = reference("cwt", lambda lib: af.CWT(num, r, 48000, wavelet_type=af.WaveletContinueType(wav), scale_type=S(scale),
+                                                  is_padding=pad, _lib=lib, **kw).cwt_planes(x))
+    re2, im2 = O.cwt(x, num, r, 48000, wav, scale, low=kw.get("low_fre", 32.703196 if scale in (5, 6) else None), is_pad=pad)
     assert rel_max(re2, re) < 1e-5 and rel_max(im2, im) < 1e-5
 
 

@@ -8,7 +8,7 @@ returned beside it meets the usual 1e-4."""
 import numpy as np
 import pytest
 
-from conftest import rel_max
+from conftest import ref_pair, rel_max
 from oracle import af_oracle as O
 
 
@@ -29,25 +29,27 @@ CASES = [(9, 16000, 1, 128, 0, 0.001, 0, 1, 0), (10, 32000, 1, 256, 0, 0.001, 1,
 
 
 @pytest.mark.parametrize("radix,sr,window,hop,re_type,thresh,pad,order,result_type", CASES)
-def test_oracle_reassign_vs_reference_build(ref_lib, radix, sr, window, hop, re_type, thresh, pad, order, result_type):
+def test_oracle_reassign_vs_reference_build(reference, radix, sr, window, hop, re_type, thresh, pad, order, result_type):
     import audioflux_b200 as af
     x = _signal(20000, sr, radix)
-    r = af.Reassign(radix, sr, af.WindowType(window), hop, af.ReassignType(re_type), thresh, bool(pad), _lib=ref_lib)
-    r.set_order(order)
-    want = r.reassign_planes(x, result_type)
+
+    def ref(lib):
+        r = af.Reassign(radix, sr, af.WindowType(window), hop, af.ReassignType(re_type), thresh, bool(pad), _lib=lib)
+        r.set_order(order)
+        return r.reassign_planes(x, result_type)
+    want = reference("planes", ref)
     got = O.reassign(x, radix, sr, window, hop, re_type, thresh, bool(pad), order, result_type)
     assert rel_max(got[2], want[2]) < 1e-4 and rel_max(got[3], want[3]) < 1e-4
     planes = (0,) if result_type else (0, 1)
     for k in planes:
-        same, fro = agree(got[k], want[k])
+        same, fro = agree(*ref_pair(got[k], want[k]))
         assert same >= 0.999 and fro <= 2e-3, (k, same, fro)
 
 
-def test_oracle_reassign_none_is_the_half_spectrum(ref_lib):
+def test_oracle_reassign_none_is_the_half_spectrum(reference):
     import audioflux_b200 as af
     x = _signal(6000, 16000, 1)
-    r = af.Reassign(9, 16000, re_type=af.ReassignType.NONE, _lib=ref_lib)
-    want = r.reassign_planes(x)
+    want = reference("planes", lambda lib: af.Reassign(9, 16000, re_type=af.ReassignType.NONE, _lib=lib).reassign_planes(x))
     got = O.reassign(x, 9, 16000, re_type=O.REASSIGN_NONE)
     assert rel_max(got[0], want[0]) < 1e-5 and rel_max(got[1], want[1]) < 1e-5
 

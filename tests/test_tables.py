@@ -7,6 +7,7 @@ import numpy as np
 import pytest
 
 import audioflux_b200 as af
+from conftest import ref_pair, ref_window
 from oracle import af_oracle as O
 
 S, ST, N, D = (af.SpectralFilterBankScaleType, af.SpectralFilterBankStyleType,
@@ -130,18 +131,22 @@ def test_cwt_tables(product_lib, wav):
     assert abs(w.get_fre_band_arr()[0] - 32.703197) < 1e-4 and abs(w.get_fre_band_arr()[83] - 3951.0667) < 1e-2
 
 
-def test_tables_against_reference_build(product_lib, ref_lib):
+def test_tables_against_reference_build(product_lib, reference):
     for wt in range(14):
-        p = ref_lib.window_calFFTWindow(wt, 2048)
-        w = np.ctypeslib.as_array(C.cast(p, C.POINTER(C.c_float)), shape=(2048,)).copy()
+        w = reference(f"window{wt}", lambda lib: ref_window(lib, wt, 2048))
         w2 = np.zeros(2048, np.float32)
         product_lib.afb200_window(wt, 2048, w2.ctypes.data)
+        w2, w = ref_pair(w2, w)
         assert np.abs(w - w2).max() < 1e-6
     for scale, style, norm in ((2, 0, 0), (2, 0, 1), (3, 1, 2), (4, 0, 0), (5, 0, 0)):
         b = af.BFT(96, 11, 44100, scale_type=S(scale), style_type=ST(style), normal_type=N(norm))
-        r = af.BFT(96, 11, 44100, scale_type=S(scale), style_type=ST(style), normal_type=N(norm), _lib=ref_lib)
-        assert np.array_equal(b.get_bin_band_arr(), r.get_bin_band_arr())
-        np.testing.assert_allclose(b.get_fre_band_arr(), r.get_fre_band_arr(), rtol=1e-6)
+
+        def bands(lib):
+            r = af.BFT(96, 11, 44100, scale_type=S(scale), style_type=ST(style), normal_type=N(norm), _lib=lib)
+            return r.get_bin_band_arr(), r.get_fre_band_arr()
+        bin_band, fre_band = reference(f"bands{scale}{style}{norm}", bands)
+        assert np.array_equal(b.get_bin_band_arr(), bin_band)
+        np.testing.assert_allclose(b.get_fre_band_arr(), fre_band, rtol=1e-6)
 
 
 def test_gammatone_bank_matches_golden_and_reference(product_lib, golden):
